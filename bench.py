@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the SoundChunks encoder hot path (DoFrame, enc:1433-1447) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the whole per-frame hot path (attenuation divider, chunk features, yakmo
@@ -23,6 +23,10 @@ searched the way the binary searches (ANN-1.1.2-style kd-tree rebuilt every pass
 encoder itself cannot be built here (DESIGN.md).  That, the cpu_baseline leg and the parity
 probe (two of the step's frames against oracle.encode_frame, outside the timed region) are the
 only places this file touches oracle/.
+
+--dump-outputs DIR (e.g. bench_outputs, which git ignores) writes what the timed path computed in
+its last step to DIR/*.npy; the inputs are seeded, so two builds run with the same arguments can
+be compared file for file (dump_outputs lists the files).
 """
 from __future__ import annotations
 
@@ -72,7 +76,54 @@ def parse_args():
     ap.add_argument("--no-lloyd", action="store_true", help="skip the secondary Lloyd-mode leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the k256 / strong_1h / split_frame legs")
     ap.add_argument("--no-parity", action="store_true", help="skip the parity probe against the oracle")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed to DIR/*.npy (rank 0; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+# ---------------------------------------------------------------------------------------------
+# outputs of the timed path, for comparing two builds run with the same arguments
+# ---------------------------------------------------------------------------------------------
+DUMP_SAMPLE_FRAMES = 16
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res, gsc=None, gsc_sizes=None):
+    """Write the per-frame results of the last timed step as float32 / float64 .npy files:
+
+      frame_scalars  float64 [F][6]            N, R, divider, passes, err, overfull of every frame
+      sample_frames  float64 [n]               a fixed, seeded sample of min(F, 16) frame numbers, ascending
+      index, attr    float32 [sum N]           the sampled frames' arrays, concatenated in that order
+      dict           float32 [sum R][chunk_size], datten float32 [sum R]   (split all four with N and R)
+      gsc_sizes      float64 [F]               .gsc size of every frame      } only when the path packs the
+      gsc_bytes      float32 [...]             the sampled frames' .gsc bytes } stream (not --impl reference)
+
+    Every frame's arrays together would exceed 64 MB at the bench shape (1,184 frames of 88,200 indexes each), so
+    they come from a sample; the scalars (the Double error sum among them) cover every frame."""
+    F = len(res)
+    pick = np.sort(np.random.default_rng(0).choice(F, min(F, DUMP_SAMPLE_FRAMES), replace=False))
+    out = {
+        "frame_scalars": np.array([[r.N, r.R, r.divider, r.passes, r.err, r.overfull] for r in res], np.float64),
+        "sample_frames": pick.astype(np.float64),
+        "index": np.concatenate([res[i].index for i in pick]).astype(np.float32),
+        "attr": np.concatenate([res[i].attr for i in pick]).astype(np.float32),
+        "dict": np.concatenate([res[i].dict for i in pick]).astype(np.float32),
+        "datten": np.concatenate([res[i].datten for i in pick]).astype(np.float32),
+    }
+    if gsc is not None:
+        offs = np.concatenate([[0], np.cumsum(gsc_sizes)])
+        b = np.frombuffer(gsc, np.uint8)
+        out["gsc_sizes"] = np.asarray(gsc_sizes, np.float64)
+        out["gsc_bytes"] = np.concatenate([b[offs[i]:offs[i + 1]] for i in pick]).astype(np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs, more than {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -187,6 +238,8 @@ def run_reference(args, rank):
     for _ in range(args.steps):
         dt, res = cpu_encode_sample(frames, args.chunks_per_frame, args.bits, cores, args.cpu_search)
         t += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     value = audio_s * args.steps / t
     sample = cpu_sample_text(cores, args.cpu_sample_seconds, res, args.chunks_per_frame, args.cpu_search)
     line = {
@@ -302,6 +355,8 @@ def main():
     res = ctx.fetch_results(layout, params)                 # also collects the stage events of the last step
     dev_stream, dev_sizes = ctx.fetch_stream(F, SAMPLE_RATE)   # .gsc bytes of the device-resident leg's last step
     stage_acc = ctx.stats()["stage_ms"]                     # last step's stage times (CUDA events, ctx stream)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, dev_stream, dev_sizes)
     passes = [r.passes for r in res]
     Ns = [r.N for r in res]
     total_audio = sum_over_ranks(audio_s_rank)
