@@ -22,6 +22,7 @@ static void usage(const char *argv0) {   // enc:1957-1981
     printf("GPU options (not in the reference):\n");
     printf("\t-gpus\tnumber of GPUs to shard frames over (default: all)\n");
     printf("\t-lloyd\tbatch Lloyd with the given iteration count instead of the reference's online rule\n");
+    printf("\t-kdtree\tsearch through the reference's ANN kd-tree (its encoder's output; -cs2 and -cs4)\n");
     printf("\n(source file must be 16bit WAV)\n\n");
 }
 

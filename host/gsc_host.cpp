@@ -119,6 +119,7 @@ extern "C" int gsch_parse_option(gsch_options *o, const char *a) {
     if (strcmp(a, "-v") == 0) { o->verbose = 1; return 0; }
     // extensions
     if (starts_with(a, "-lloyd")) { o->kmeans_mode = 1; o->lloyd_iters = (int)param_value(a, "-lloyd", o->lloyd_iters); return 0; }
+    if (strcmp(a, "-kdtree") == 0) { o->kmeans_mode = 3; return 0; }
     if (starts_with(a, "-gpus")) { o->devices = (int)param_value(a, "-gpus", o->devices); return 0; }
     return 1;
 }

@@ -146,6 +146,13 @@ int gsc_knn_scan_reduce(gsc_ctx *ctx, const float *X, int N, int D,
                         float *centroids, int K, int precision, int max_passes,
                         int32_t *labels, int *passes, double *err);
 
+/* kmeans_mode 3: enc:699-765 with the search the reference binary performs -- an ANN 1.1.2 kd-tree over the
+ * centroids, rebuilt at the start of every pass (planes and boxes from the pass start, leaves read the live rows,
+ * ties to the first point visited).  Bit-identical to the oracle's kd-tree rule.  D in {4, 8},
+ * 1 <= K <= 4096.  Same arguments as gsc_knn_scan_reduce. */
+int gsc_knn_scan_reduce_kdtree(gsc_ctx *ctx, const float *X, int N, int D, float *centroids, int K, int precision,
+                               int max_passes, int32_t *labels, int *passes, double *err);
+
 /* Plain batch Lloyd (BASELINE.json's 1e-4 centroid contract): `iters` x
  * (exact assign, mean), then a final assign.  centroids in/out.  Member rows
  * are accumulated in Double and the mean is rounded to Single once: two
@@ -209,6 +216,12 @@ int gsc_knnfit(gsc_ctx *ctx, const int16_t *dict, const uint8_t *datten, int R,
                int64_t stride, int C, int S, int32_t *best, int32_t *use,
                int32_t *band);
 
+/* kmeans_mode 3: enc:915-965 the way the binary runs it -- an ANN kd-tree over the 4R variant rows, the 64 nearest
+ * rows per chunk (standard search, ties in visit order), the lowest row index within epsilon of the nearest.
+ * Bit-identical to the oracle's kd-tree KNNFit.  best int32[N] (variant row), use int32[R]. */
+int gsc_knnfit_kdtree(gsc_ctx *ctx, const int16_t *dict, const uint8_t *datten, int R, int cs, int bits, int divider,
+                      const int16_t *pcm, int64_t stride, int C, int S, int32_t *best, int32_t *use);
+
 /* enc:970-977: prune unused entries, sort by use count (FreePascal quicksort
  * order), renumber.  remap int32[R] old->new or -1; order int32[R]. */
 int gsc_finalize_dictionary(gsc_ctx *ctx, const int32_t *use, int R,
@@ -224,7 +237,9 @@ typedef struct gsc_params {
     int32_t chunks_per_frame;  /* -cpf  enc:1505 (<=4096) */
     int32_t precision;         /* -pr   enc:1503 (3); 0 = passthrough */
     int32_t max_passes;        /* CMaxIterations enc:703 (100) */
-    int32_t kmeans_mode;       /* 0 online (reference rule), 1 Lloyd */
+    int32_t kmeans_mode;       /* 0 online (reference rule, exact search), 1 Lloyd,
+                                  3 online through the reference's ANN kd-tree searches (k-means and KNNFit;
+                                  chunk sizes 2 and 4) */
     int32_t lloyd_iters;       /* mode 1 */
     int32_t reserved;
 } gsc_params;
@@ -289,12 +304,14 @@ int gsc_fetch_quality(gsc_ctx *ctx, int n_frames, uint64_t *sq_err, int64_t *sam
 #define GSC_DBG_ONLINE_BATCHED 32u /* K <= 256: the batched CTA-per-frame kernel instead of the warp-per-frame one */
 #define GSC_DBG_LABEL_SCAN     64u /* per-cluster sums by scanning all labels per cluster (O(K*N)) instead of member lists */
 #define GSC_DBG_DIVIDER_V1     128u /* FindAttenuationDivider with the per-thread loop that divides in the inner loop */
+#define GSC_DBG_KDTREE_SERIAL  256u /* kmeans_mode 3: the kd-tree k-means searches one point per round (no speculation) */
 int gsc_ctx_set_debug(gsc_ctx *ctx, unsigned flags);
 /* Exhaustive self-check of the tabulated-reciprocal division used by the attenuation-divider kernel at `bits`. */
 int gsc_selftest_divider_division(gsc_ctx *ctx, int bits, uint64_t *mismatches);
 /* Debug: counters of the last online k-means launch, 16 x uint64 per frame:
  * batches, points, re-filtered points, resolver rounds, full candidate lists,
- * candidates (lane 0); rest reserved (zero). */
+ * candidates (lane 0); rest reserved (zero).  After a kmeans_mode 3 k-means (all passes):
+ * speculation rounds, points committed, lane searches, visit lists that overflowed. */
 int gsc_debug_online_counters(gsc_ctx *ctx, unsigned long long *out, int n_frames);
 /* Debug: counters of the last seeding launch, 8 x uint64 per frame: cycles of seed pick, distance pass,
  * summaries + chain, number of steps; windows evaluated exactly, blocks visited, windows re-summarised, chain cycles. */

@@ -46,7 +46,8 @@ typedef struct gsch_options {
     int32_t chunk_blend;        /* -cb   enc:1500 (0)     must stay 0           */
     int32_t verbose;            /* -v                                           */
     /* not in the reference CLI */
-    int32_t kmeans_mode;        /* 0 online rule (reference), 1 batch Lloyd     */
+    int32_t kmeans_mode;        /* 0 online rule (reference), 1 batch Lloyd (-lloyd),
+                                   3 reference's kd-tree searches (-kdtree)     */
     int32_t lloyd_iters;
     int32_t max_passes;         /* CMaxIterations enc:703 (100)                 */
     int32_t devices;            /* GPUs to shard frames over, 0 = all visible   */

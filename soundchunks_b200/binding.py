@@ -24,9 +24,9 @@ EXPORTS = [
     "ann_kdtree_search_multi", "ann_kdtree_pri_search_multi",
     "gsc_last_error", "gsc_device_count", "gsc_create", "gsc_destroy", "gsc_ctx_device", "gsc_ctx_stream",
     "gsc_synchronize", "gsc_get_stats", "gsc_stage_busy_ms", "gsc_reset_stats",
-    "gsc_find_attenuation_divider", "gsc_make_chunks", "gsc_yakmo", "gsc_knn_scan_reduce", "gsc_lloyd",
+    "gsc_find_attenuation_divider", "gsc_make_chunks", "gsc_yakmo", "gsc_knn_scan_reduce", "gsc_knn_scan_reduce_kdtree", "gsc_lloyd",
     "gsc_assign", "gsc_split_begin", "gsc_split_step", "gsc_split_update", "gsc_split_end",
-    "gsc_split_unique_id", "gsc_split_comm_init", "gsc_split_comm_destroy", "gsc_split_seed", "gsc_split_lloyd", "gsc_build_dictionary", "gsc_knnfit", "gsc_finalize_dictionary",
+    "gsc_split_unique_id", "gsc_split_comm_init", "gsc_split_comm_destroy", "gsc_split_seed", "gsc_split_lloyd", "gsc_build_dictionary", "gsc_knnfit", "gsc_knnfit_kdtree", "gsc_finalize_dictionary",
     "gsc_default_params", "gsc_dict_capacity", "gsc_encode_frames", "gsc_encode_frames_dev",
     "gsc_fetch_results", "gsc_fetch_stream", "gsc_fetch_quality", "gsc_fp32_peak_probe", "gsc_log_array", "gsc_plan_frames", "gsc_plan_frames_dev", "gsc_ctx_set_debug", "gsc_selftest_divider_division", "gsc_debug_online_counters", "gsc_debug_seed_counters",
 ]
@@ -201,6 +201,7 @@ class Context:
         return out
 
     DBG_ONLINE_EXACT, DBG_SEED_FULLSCAN, DBG_SEED_SERIAL, DBG_KNNFIT_DENSE, DBG_LLOYD_OWNER, DBG_ONLINE_BATCHED, DBG_LABEL_SCAN, DBG_DIVIDER_V1 = 1, 2, 4, 8, 16, 32, 64, 128
+    DBG_KDTREE_SERIAL = 256
 
     def set_debug(self, flags: int):
         """Cross-check paths (include/gsc_cuda.h GSC_DBG_*); 0 = the product path."""
@@ -284,6 +285,18 @@ class Context:
         err = C.c_double(0)
         self._ck(self.L.gsc_knn_scan_reduce(C.c_void_p(self.h), _vp(X), N, D, _vp(cen), cen.shape[0], precision,
                                             max_passes, _vp(labels), C.byref(passes), C.byref(err)))
+        return cen, labels, passes.value, err.value
+
+    def knn_scan_reduce_kdtree(self, X, centroids, precision=3, max_passes=100):
+        """kmeans_mode 3: KNNScanReduce through the reference's ANN kd-tree -> (centroids, labels, passes, err)"""
+        X = np.ascontiguousarray(X, dtype=np.float32)
+        cen = np.array(centroids, dtype=np.float32, order="C", copy=True)
+        N, D = X.shape
+        labels = np.zeros(N, np.int32)
+        passes = C.c_int(0)
+        err = C.c_double(0)
+        self._ck(self.L.gsc_knn_scan_reduce_kdtree(C.c_void_p(self.h), _vp(X), N, D, _vp(cen), cen.shape[0], precision,
+                                                   max_passes, _vp(labels), C.byref(passes), C.byref(err)))
         return cen, labels, passes.value, err.value
 
     def lloyd(self, X, centroids, iters):
@@ -379,6 +392,19 @@ class Context:
         out = dict(best=np.zeros(N, np.int32), use=np.zeros(R, np.int32), band=np.zeros(N, np.int32))
         self._ck(self.L.gsc_knnfit(C.c_void_p(self.h), _vp(dic), _vp(datten), R, cs, bits, divider, _vp(pcm),
                                    C.c_int64(S), Cn, S, _vp(out["best"]), _vp(out["use"]), _vp(out["band"])))
+        return out
+
+    def knnfit_kdtree(self, dic, datten, pcm, cs=4, bits=12, divider=6):
+        """kmeans_mode 3: KNNFit through the reference's ANN kd-tree (64 nearest rows) -> dict(best, use)"""
+        pcm = _pcm(pcm)
+        Cn, S = pcm.shape
+        dic = np.ascontiguousarray(dic, dtype=np.int16)
+        datten = np.ascontiguousarray(datten, dtype=np.uint8)
+        R = dic.shape[0]
+        N = ((S - 1) // cs + 1) * Cn
+        out = dict(best=np.zeros(N, np.int32), use=np.zeros(R, np.int32))
+        self._ck(self.L.gsc_knnfit_kdtree(C.c_void_p(self.h), _vp(dic), _vp(datten), R, cs, bits, divider, _vp(pcm),
+                                          C.c_int64(S), Cn, S, _vp(out["best"]), _vp(out["use"])))
         return out
 
     def finalize_dictionary(self, use):

@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libgsc_cuda.so")
 SOURCES = ["gsc_api.cu"]
-DEPS = ["gsc_api.cu", "gsc_kernels.cuh", "gsc_online.cuh", "gsc_device.cuh", os.path.join("..", "..", "include", "gsc_cuda.h")]
+DEPS = ["gsc_api.cu", "gsc_kernels.cuh", "gsc_online.cuh", "gsc_kdtree.cuh", "gsc_device.cuh", os.path.join("..", "..", "include", "gsc_cuda.h")]
 
 
 def nvcc_path() -> str:

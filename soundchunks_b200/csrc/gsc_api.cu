@@ -25,6 +25,7 @@
 #include "gsc_seed.cuh"
 #include "gsc_online.cuh"
 #include "gsc_plan.cuh"
+#include "gsc_kdtree.cuh"
 
 // ---------------------------------------------------------------------------
 // error handling, FP environment
@@ -125,6 +126,7 @@ struct gsc_ctx {
         sums, cnt0, labels, passes, err, means0, means, order, counts, dict, datten, dattr, entry, best,
         use, band, overfull, remap, order2, newR, odict, odatten, oindex, oattr, dist, misc, dbg, sdbg, kv, kn, ke, sbytes, snb, sqerr,
         perm, pns, xs, blo, bhi, wsum, cstate, odone, members, moffs, cenh,
+        kcnt, ktv, ktn, ktp, ktd, ktb,
         pl_terms, pl_wsum, pl_wpre, pl_win, pl_scal, pl_starts, pl_next;
     void *nccl_comm = nullptr;       // ncclComm_t of the oversized-frame split (gsc_split_comm_init)
     int nccl_ranks = 1, nccl_rank = 0;
@@ -208,6 +210,7 @@ extern "C" void gsc_destroy(gsc_ctx *c) {
                       &c->datten, &c->dattr, &c->entry, &c->best, &c->use, &c->band, &c->overfull, &c->remap,
                       &c->order2, &c->newR, &c->odict, &c->odatten, &c->oindex, &c->oattr, &c->dist, &c->misc, &c->dbg, &c->sdbg, &c->kv, &c->kn, &c->ke, &c->sbytes, &c->snb, &c->sqerr, &c->scompact, &c->soffs,
                       &c->perm, &c->pns, &c->xs, &c->blo, &c->bhi, &c->wsum, &c->cstate, &c->odone, &c->members, &c->moffs, &c->cenh,
+                      &c->kcnt, &c->ktv, &c->ktn, &c->ktp, &c->ktd, &c->ktb,
                       &c->pl_terms, &c->pl_wsum, &c->pl_wpre, &c->pl_win, &c->pl_scal, &c->pl_starts, &c->pl_next};
     for (DevBuf *b : bufs) b->release();
     c->hsizes.release();
@@ -636,6 +639,53 @@ static int stage_online(gsc_ctx *c, int D, int precision, int max_passes) {
         if (K <= 4096) return online_launch<4, 16, 256>(c, tol, max_passes, fe);
     }
     return set_err(GSC_ERR_UNSUPPORTED, "online k-means supports D in {4, 8} and K <= 4096 (got D=%d K=%d)", D, K);
+}
+
+// kmeans_mode 3: KNNScanReduce through the ANN kd-tree (gsc_kdtree.cuh), one CTA per frame.  Counters (online counter
+// buffer, 16 x uint64 per frame): speculation rounds, points committed, lane searches, overflowed visit lists.
+static int stage_kdtree_scan(gsc_ctx *c, int D, int precision, int max_passes) {
+    if (D != 4 && D != 8)
+        return set_err(GSC_ERR_UNSUPPORTED, "kd-tree k-means supports D in {4, 8} (got D=%d)", D);
+    TRY(c->passes.ensure(4 * (size_t)c->F)); TRY(c->err.ensure(8 * (size_t)c->F));
+    TRY(c->dbg.ensure(128 * (size_t)c->F)); TRY(c->kcnt.ensure(4 * (size_t)c->F * c->Kmax));
+    CU(cudaMemsetAsync(c->passes.p, 0, 4 * (size_t)c->F, c->stream));
+    CU(cudaMemsetAsync(c->err.p, 0, 8 * (size_t)c->F, c->stream));
+    CU(cudaMemsetAsync(c->dbg.p, 0, 128 * (size_t)c->F, c->stream));
+    const double tol = int_power10_neg(precision);
+    const int lanes = (c->debug & GSC_DBG_KDTREE_SERIAL) ? 1 : 32;
+    const size_t smem = GscKdtScanSmem(c->Kmax, D).total;
+#define GSC_KDT_LAUNCH(DD)                                                                                             \
+    do {                                                                                                               \
+        SMEM_OPTIN(k_kdt_scan<DD>, smem);                                                                              \
+        LAUNCH(c, k_kdt_scan<DD>, c->F, GSC_KDT_THREADS, smem, c->frames.as<GscFrame>(), c->feat.as<float>(),          \
+               c->cen.as<float>(), c->labels.as<int>(), c->passes.as<int>(), c->err.as<double>(), c->kcnt.as<int>(),  \
+               tol, max_passes, c->Kmax, lanes, c->dbg.as<unsigned long long>());                                      \
+    } while (0)
+    if (D == 8) GSC_KDT_LAUNCH(8); else GSC_KDT_LAUNCH(4);
+#undef GSC_KDT_LAUNCH
+    return GSC_OK;
+}
+
+// kmeans_mode 3: KNNFit through a kd-tree over every frame's 4R variant rows (build, then one thread per query).
+// Band populations are not computed in this mode: overfull stays 0.
+static int stage_kdtree_fit(gsc_ctx *c) {
+    const int cs = c->cs;
+    const size_t fk = (size_t)c->F * c->Kmax, fm = 4 * fk;
+    TRY(c->best.ensure(4 * (size_t)c->sumN)); TRY(c->use.ensure(4 * fk)); TRY(c->overfull.ensure(4 * (size_t)c->F));
+    TRY(c->ktv.ensure(4 * fm * cs)); TRY(c->ktn.ensure(4 * 3 * fm)); TRY(c->ktp.ensure(2 * fm)); TRY(c->ktd.ensure(fm));
+    TRY(c->ktb.ensure(4 * 2 * (size_t)c->F * cs));
+    CU(cudaMemsetAsync(c->use.p, 0, 4 * fk, c->stream));
+    CU(cudaMemsetAsync(c->overfull.p, 0, 4 * (size_t)c->F, c->stream));
+    dim3 grid((c->maxN + 127) / 128, c->F);
+    DISPATCH_CS(cs, {
+        LAUNCH(c, k_kdt_fit_build<CS>, c->F, 256, 0, c->frames.as<GscFrame>(), c->bits, c->divider.as<int>(),
+               c->dict.as<short>(), c->datten.as<unsigned char>(), c->ktv.as<float>(), c->ktn.as<float>(),
+               c->ktp.as<unsigned short>(), c->ktd.as<unsigned char>(), c->ktb.as<float>(), c->Kmax);
+        LAUNCH(c, k_kdt_fit<CS>, grid, 128, 0, c->frames.as<GscFrame>(), c->pcm.as<short>(), c->bits, c->divider.as<int>(),
+               c->ktv.as<float>(), c->ktn.as<float>(), c->ktp.as<unsigned short>(), c->ktd.as<unsigned char>(),
+               c->ktb.as<float>(), c->best.as<int>(), c->use.as<int>(), c->Kmax);
+    });
+    return GSC_OK;
 }
 
 static int stage_dictionary(gsc_ctx *c, bool want_entry) {
@@ -1124,6 +1174,46 @@ extern "C" int gsc_knnfit(gsc_ctx *c, const int16_t *dict, const uint8_t *datten
     return sync(c);
 }
 
+extern "C" int gsc_knn_scan_reduce_kdtree(gsc_ctx *c, const float *X, int N, int D, float *centroids, int K, int precision,
+                                          int max_passes, int32_t *labels, int *passes, double *err) {
+    FpGuard g;
+    if (!c || !centroids) return set_err(GSC_ERR_ARG, "null argument");
+    if (max_passes < 1) return set_err(GSC_ERR_ARG, "max_passes must be >= 1");
+    if (D != 4 && D != 8) return set_err(GSC_ERR_UNSUPPORTED, "kd-tree k-means supports D in {4, 8} (got D=%d)", D);
+    TRY(upload_points(c, X, N, D, K));
+    TRY(c->cen.ensure(4 * (size_t)K * D)); TRY(c->labels.ensure(4 * (size_t)N));
+    TRY(h2d(c, c->cen.p, centroids, 4 * (size_t)K * D));
+    TRY(stage_kdtree_scan(c, D, precision, max_passes));
+    TRY(d2h(c, centroids, c->cen.p, 4 * (size_t)K * D));
+    if (labels) TRY(d2h(c, labels, c->labels.p, 4 * (size_t)N));
+    int p = 0; double e = 0;
+    TRY(d2h(c, &p, c->passes.p, 4)); TRY(d2h(c, &e, c->err.p, 8));
+    TRY(sync(c));
+    if (passes) *passes = p;
+    if (err) *err = e;
+    return GSC_OK;
+}
+
+extern "C" int gsc_knnfit_kdtree(gsc_ctx *c, const int16_t *dict, const uint8_t *datten, int R, int cs, int bits, int divider,
+                                 const int16_t *pcm, int64_t stride, int C, int S, int32_t *best, int32_t *use) {
+    FpGuard g;
+    TRY(check_common(c, cs, bits));
+    if (!dict || !datten || R <= 0 || R > GSC_MAX_K || divider < 1) return set_err(GSC_ERR_ARG, "bad arguments");
+    TRY(single_frame_pcm(c, pcm, stride, C, S, cs, bits, R, 1));
+    GscFrame &f = c->h_frames[0];
+    f.K = R; f.R = R;
+    c->Kmax = R;
+    TRY(upload_frames(c));
+    TRY(c->dict.ensure(2 * (size_t)R * cs)); TRY(c->datten.ensure(R)); TRY(c->divider.ensure(4));
+    TRY(h2d(c, c->dict.p, dict, 2 * (size_t)R * cs));
+    TRY(h2d(c, c->datten.p, datten, R));
+    TRY(h2d(c, c->divider.p, &divider, 4));
+    TRY(stage_kdtree_fit(c));
+    if (best) TRY(d2h(c, best, c->best.p, 4 * (size_t)c->sumN));
+    if (use) TRY(d2h(c, use, c->use.p, 4 * (size_t)R));
+    return sync(c);
+}
+
 extern "C" int gsc_finalize_dictionary(gsc_ctx *c, const int32_t *use, int R, int32_t *remap, int32_t *order,
                                        int *new_R) {
     FpGuard g;
@@ -1159,6 +1249,8 @@ static int check_params(const gsc_params *p) {
     if (p->chunk_bit_depth != 8 && p->chunk_bit_depth != 12)
         return set_err(GSC_ERR_ARG, "chunk_bit_depth must be 8 or 12 (enc:1041)");
     if (p->max_passes < 1) return set_err(GSC_ERR_ARG, "max_passes must be >= 1");
+    if (p->kmeans_mode == 3 && p->chunk_size == 8)
+        return set_err(GSC_ERR_UNSUPPORTED, "kmeans_mode 3 supports chunk sizes 2 and 4");
     return GSC_OK;
 }
 
@@ -1184,6 +1276,8 @@ static int run_pipeline(gsc_ctx *c, const gsc_params *P) {
             TRY(c->passes.ensure(4 * (size_t)c->F)); TRY(c->err.ensure(8 * (size_t)c->F));
             CU(cudaMemsetAsync(c->passes.p, 0, 4 * (size_t)c->F, c->stream));
             CU(cudaMemsetAsync(c->err.p, 0, 8 * (size_t)c->F, c->stream));
+        } else if (P->kmeans_mode == 3) {
+            TRY(stage_kdtree_scan(c, D, P->precision, P->max_passes));   // enc:835 through the kd-tree
         } else {
             // first-pass guesses: the seed cell of every point
             CU(cudaMemcpyAsync(c->labels.p, c->sid.p, 4 * (size_t)c->sumN, cudaMemcpyDeviceToDevice, c->stream));
@@ -1197,7 +1291,8 @@ static int run_pipeline(gsc_ctx *c, const gsc_params *P) {
     CU(cudaEventRecord(c->ev[4], c->stream));
     TRY(stage_dictionary(c, false));                                // enc:843-889
     CU(cudaEventRecord(c->ev[5], c->stream));
-    TRY(stage_knnfit(c, false));                                    // enc:1443
+    if (P->kmeans_mode == 3) TRY(stage_kdtree_fit(c));              // enc:1443 through the kd-tree
+    else TRY(stage_knnfit(c, false));                               // enc:1443
     CU(cudaEventRecord(c->ev[6], c->stream));
     TRY(stage_finalize(c, true));                                   // enc:970-977
     CU(cudaEventRecord(c->ev[7], c->stream));
