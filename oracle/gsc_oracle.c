@@ -446,14 +446,14 @@ static void dist_all(const float *q, const float *Ct, int Kp, int K, int D,
     }
 }
 
+/* strict <: lowest index on ties, NaN distances never win; every distance NaN (an all-NaN codebook) -> centroid 0
+ * at d = +inf, what the kernels report */
 static inline int argmin_first(const float *acc, int K, float *bd)
 {
     int best = 0;
     float b = INFINITY;
-    int found = 0;
     for (int k = 0; k < K; ++k)
-        if (acc[k] < b) { b = acc[k]; best = k; found = 1; }
-    if (!found) b = acc[0];
+        if (acc[k] < b) { b = acc[k]; best = k; }
     *bd = b;
     return best;
 }

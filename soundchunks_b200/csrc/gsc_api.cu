@@ -141,8 +141,10 @@ struct gsc_ctx {
     int batch_total = 0;             // frames of the batch in flight over both lanes (0: single-stage call)
     std::vector<int> idx_a, idx_b;   // frames of the last split batch handled by this context / by the peer
     double stage_t[8] = {};          // start of stage i (ev[i]) in ms after the batch's fork event, filled at fetch
-    // .gsc stream of the last batch: packed once (k_pack_frames), sizes kept for the second gsc_fetch_stream call
+    // .gsc stream of the last batch: packed once per sample rate (k_pack_frames; the rate is in every frame header),
+    // sizes kept for the second gsc_fetch_stream call
     bool packed = false;
+    int packed_rate = 0;
     std::vector<long long> pk_sizes;  // bytes per frame of this lane
     DevBuf scompact, soffs;           // main context: the batch's frames back to back in frame order; per-lane offsets
     HostBuf hsizes;
@@ -743,7 +745,7 @@ static int stage_knnfit(gsc_ctx *c, bool want_band) {
         });
         return GSC_OK;
     }
-    size_t smem = sizeof(float) * (size_t)c->Kmax * cs;
+    size_t smem = sizeof(float) * (size_t)c->Kmax * (cs + 1);
     DISPATCH_CS(cs, {
         SMEM_OPTIN(k_knnfit<CS>, smem);
         LAUNCH(c, k_knnfit<CS>, grid, 256, smem, c->frames.as<GscFrame>(), c->pcm.as<short>(), c->bits,
@@ -1414,11 +1416,11 @@ static long long stream_cap(const gsc_ctx *c) {   // bytes per frame slot, multi
     const long long v = 12 + (c->Kmax + 1) / 2 + 2LL * c->Kmax * c->cs + 4 + 2 * ((17LL * c->maxN + 15) / 16) + 8;
     return (v + 3) & ~3LL;
 }
-// k_pack_frames for one lane's frames (once per batch) + its per-frame sizes on the host
+// k_pack_frames for one lane's frames (once per batch and sample rate) + its per-frame sizes on the host
 static int pack_lane(gsc_ctx *c, int sample_rate) {
     CU(cudaSetDevice(c->device));
     const long long cap = stream_cap(c);
-    if (!c->packed) {
+    if (!c->packed || c->packed_rate != sample_rate) {
         TRY(c->sbytes.ensure((size_t)cap * c->F)); TRY(c->snb.ensure(8 * (size_t)c->F));
         DISPATCH_CS(c->cs, LAUNCH(c, k_pack_frames<CS>, c->F, 1024, 0, c->frames.as<GscFrame>(), c->bits, sample_rate,
                                   c->divider.as<int>(), c->newR.as<int>(), c->odict.as<short>(), c->odatten.as<unsigned char>(),
@@ -1429,6 +1431,7 @@ static int pack_lane(gsc_ctx *c, int sample_rate) {
         TRY(sync(c));                                        // the sizes are read on the host right below
         c->pk_sizes.assign(c->hsizes.as<long long>(), c->hsizes.as<long long>() + c->F);
         c->packed = true;
+        c->packed_rate = sample_rate;
     }
     return GSC_OK;
 }

@@ -1144,18 +1144,40 @@ __device__ __forceinline__ bool gsc_in_band(float a, float d, float fcs, float e
     return (a > b) ? ((a - b) <= eps) : ((b - a) <= eps);  // SameValue(Single)
 }
 
+// Bit j set: component j of the entry is -32768, whose sign image is itself (enc:1665-1680 negates a SmallInt with
+// range checks off), so the negated variants keep +v there instead of -v.
 template <int CS>
-__device__ __forceinline__ void gsc_variant_dists(const float (&q)[CS], const float (&v)[CS],
+__device__ __forceinline__ unsigned gsc_min16_mask(const short *e) {
+    unsigned m = 0;
+#pragma unroll
+    for (int j = 0; j < CS; ++j) m |= (e[j] == (short)-32768) ? (1u << j) : 0u;
+    return m;
+}
+
+template <int CS>
+__device__ __forceinline__ void gsc_variant_dists(const float (&q)[CS], const float (&v)[CS], unsigned m,
                                                   float &d0, float &d1, float &d2, float &d3) {
     d0 = 0.0f; d1 = 0.0f; d2 = 0.0f; d3 = 0.0f;
+    if (m == 0) {
 #pragma unroll
-    for (int j = 0; j < CS; ++j) {
-        float t0 = q[j] - v[j];
-        float t1 = q[j] - v[CS - 1 - j];
-        float t2 = q[j] + v[j];
-        float t3 = q[j] + v[CS - 1 - j];
-        float m0 = t0 * t0, m1 = t1 * t1, m2 = t2 * t2, m3 = t3 * t3;
-        d0 = d0 + m0; d1 = d1 + m1; d2 = d2 + m2; d3 = d3 + m3;
+        for (int j = 0; j < CS; ++j) {
+            float t0 = q[j] - v[j];
+            float t1 = q[j] - v[CS - 1 - j];
+            float t2 = q[j] + v[j];
+            float t3 = q[j] + v[CS - 1 - j];
+            float m0 = t0 * t0, m1 = t1 * t1, m2 = t2 * t2, m3 = t3 * t3;
+            d0 = d0 + m0; d1 = d1 + m1; d2 = d2 + m2; d3 = d3 + m3;
+        }
+    } else {
+#pragma unroll
+        for (int j = 0; j < CS; ++j) {
+            float t0 = q[j] - v[j];
+            float t1 = q[j] - v[CS - 1 - j];
+            float t2 = ((m >> j) & 1u) ? q[j] - v[j] : q[j] + v[j];
+            float t3 = ((m >> (CS - 1 - j)) & 1u) ? q[j] - v[CS - 1 - j] : q[j] + v[CS - 1 - j];
+            float m0 = t0 * t0, m1 = t1 * t1, m2 = t2 * t2, m3 = t3 * t3;
+            d0 = d0 + m0; d1 = d1 + m1; d2 = d2 + m2; d3 = d3 + m3;
+        }
     }
 }
 
@@ -1179,11 +1201,12 @@ __global__ void __launch_bounds__(256) k_knnfit(const GscFrame *__restrict__ fra
                                                 int *__restrict__ band,      // [sumN] or null
                                                 int *__restrict__ overfull,  // [F], zeroed
                                                 int Kmax) {
-    extern __shared__ float s_v[];  // [R][CS]
+    extern __shared__ float s_v[];  // [R][CS] | [R] -32768 masks (as unsigned)
     const GscFrame f = frames[blockIdx.y];
     if ((long long)blockIdx.x * blockDim.x >= f.N) return;
     const long long fo = (long long)f.slot * Kmax;
     const int R = f.R;
+    unsigned *s_m = reinterpret_cast<unsigned *>(s_v + (size_t)R * CS);
     const double law = 1.0 / (double)divider[f.slot];
     GscLaw L;
     L.init(law);
@@ -1192,6 +1215,7 @@ __global__ void __launch_bounds__(256) k_knnfit(const GscFrame *__restrict__ fra
         const int e = t / CS;
         s_v[t] = (float)gsc_dequant(dict[fo * CS + t], obd, L.T[datten[fo + e]], false);  // enc:932
     }
+    for (int e = threadIdx.x; e < R; e += blockDim.x) s_m[e] = gsc_min16_mask<CS>(dict + (fo + e) * CS);
     __syncthreads();
     const int n = blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= f.N) return;
@@ -1208,7 +1232,7 @@ __global__ void __launch_bounds__(256) k_knnfit(const GscFrame *__restrict__ fra
 #pragma unroll
         for (int j = 0; j < CS; ++j) v[j] = s_v[e * CS + j];
         float d0, d1, d2, d3;
-        gsc_variant_dists<CS>(q, v, d0, d1, d2, d3);
+        gsc_variant_dists<CS>(q, v, s_m[e], d0, d1, d2, d3);
         dmin = fminf(dmin, fminf(fminf(d0, d1), fminf(d2, d3)));
     }
     // threshold: largest float d with in_band(d)
@@ -1228,7 +1252,7 @@ __global__ void __launch_bounds__(256) k_knnfit(const GscFrame *__restrict__ fra
 #pragma unroll
         for (int j = 0; j < CS; ++j) v[j] = s_v[e * CS + j];
         float d0, d1, d2, d3;
-        gsc_variant_dists<CS>(q, v, d0, d1, d2, d3);
+        gsc_variant_dists<CS>(q, v, s_m[e], d0, d1, d2, d3);
         const bool b0 = d0 <= dthr, b1 = d1 <= dthr, b2 = d2 <= dthr, b3 = d3 <= dthr;
         if (b0 | b1 | b2 | b3) {
             nb += (int)b0 + (int)b1 + (int)b2 + (int)b3;
@@ -1263,7 +1287,7 @@ __global__ void __launch_bounds__(256) k_knn_prep(const GscFrame *__restrict__ f
                                                   const unsigned char *__restrict__ datten,
                                                   float *__restrict__ sV,   // [F][Kmax][CS] base variants, norm order
                                                   float *__restrict__ sN,   // [F][Kmax] norms, ascending
-                                                  int *__restrict__ sE,     // [F][Kmax] entry of each position
+                                                  int *__restrict__ sE,     // [F][Kmax] entry | -32768 mask << 24
                                                   int Kmax) {
     extern __shared__ unsigned long long s_key[];   // [R2] (norm bits << 32 | entry)
     const GscFrame f = frames[blockIdx.x];
@@ -1303,7 +1327,7 @@ __global__ void __launch_bounds__(256) k_knn_prep(const GscFrame *__restrict__ f
         const unsigned long long key = s_key[p];
         const int e = (int)(key & 0xffffffffu);
         sN[fo + p] = __uint_as_float((unsigned)(key >> 32));
-        sE[fo + p] = e;
+        sE[fo + p] = e | (int)(gsc_min16_mask<CS>(dict + (fo + e) * CS) << 24);   // e < GSC_MAX_K < 2^24
 #pragma unroll
         for (int j = 0; j < CS; ++j)
             sV[(fo + p) * CS + j] = (float)gsc_dequant(dict[(fo + e) * CS + j], obd, L.T[datten[fo + e]], false);   // enc:932
@@ -1358,7 +1382,7 @@ __global__ void __launch_bounds__(256) k_knnfit_win(const GscFrame *__restrict__
 #pragma unroll
                     for (int j = 0; j < CS; ++j) v[j] = s_v[up * CS + j];
                     float d0, d1, d2, d3;
-                    gsc_variant_dists<CS>(q, v, d0, d1, d2, d3);
+                    gsc_variant_dists<CS>(q, v, (unsigned)s_e[up] >> 24, d0, d1, d2, d3);
                     dmin = fminf(dmin, fminf(fminf(d0, d1), fminf(d2, d3)));
                     upok = ++up < R;
                 }
@@ -1370,7 +1394,7 @@ __global__ void __launch_bounds__(256) k_knnfit_win(const GscFrame *__restrict__
 #pragma unroll
                     for (int j = 0; j < CS; ++j) v[j] = s_v[dn * CS + j];
                     float d0, d1, d2, d3;
-                    gsc_variant_dists<CS>(q, v, d0, d1, d2, d3);
+                    gsc_variant_dists<CS>(q, v, (unsigned)s_e[dn] >> 24, d0, d1, d2, d3);
                     dmin = fminf(dmin, fminf(fminf(d0, d1), fminf(d2, d3)));
                     dnok = --dn >= 0;
                 }
@@ -1398,11 +1422,11 @@ __global__ void __launch_bounds__(256) k_knnfit_win(const GscFrame *__restrict__
 #pragma unroll
             for (int j = 0; j < CS; ++j) v[j] = s_v[p * CS + j];
             float d0, d1, d2, d3;
-            gsc_variant_dists<CS>(q, v, d0, d1, d2, d3);
+            gsc_variant_dists<CS>(q, v, (unsigned)s_e[p] >> 24, d0, d1, d2, d3);
             const bool b0 = d0 <= dthr, b1 = d1 <= dthr, b2 = d2 <= dthr, b3 = d3 <= dthr;
             if (b0 | b1 | b2 | b3) {
                 nb += (int)b0 + (int)b1 + (int)b2 + (int)b3;
-                const int r0 = s_e[p] * 4 + (b0 ? 0 : b1 ? 1 : b2 ? 2 : 3);
+                const int r0 = (s_e[p] & 0xffffff) * 4 + (b0 ? 0 : b1 ? 1 : b2 ? 2 : 3);
                 bi = min(bi, r0);
             }
             p += dir ? -1 : 1;

@@ -61,9 +61,9 @@ def test_make_chunks(ctx, oracle):
         assert np.array_equal(g_feat.view(np.uint32), feat.view(np.uint32))
 
 
-def _features(oracle, seconds=0.5, ch=1, seed=11, sr=44100):
+def _features(oracle, seconds=0.5, ch=1, seed=11, sr=44100, cs=4):
     pcm = _quiet(_audio(seconds, sr, ch, seed))
-    raw, attr, atten, feat, dst = oracle.make_chunks(pcm, 4, 12, 6)
+    raw, attr, atten, feat, dst = oracle.make_chunks(pcm, cs, 12, 6)
     return pcm, raw, attr, feat
 
 
@@ -146,16 +146,30 @@ def test_yakmo_random_init_and_iters(ctx, oracle):
     assert np.array_equal(l_gpu, l_ref)
 
 
-@pytest.mark.parametrize("K,seconds,passes", [(256, 0.25, 100), (100, 0.1, 7), (4096, 0.6, 4), (700, 0.3, 20), (1500, 0.4, 8), (400, 0.2, 12)])
-def test_online_kmeans_bit_exact(ctx, oracle, K, seconds, passes):
-    pcm, raw, attr, feat = _features(oracle, seconds, ch=2 if K == 4096 else 1)
+# D = 8 (-cs 4) and D = 4 (-cs 2, its own features): both sides of every CTA-shape bucket of k_online (gsc_api.cu
+# stage_online: K <= 256 / 512 / 1024 / 2048 / 4096)
+ONLINE_CASES = [(256, 0.25, 100, 8), (100, 0.1, 7, 8), (4096, 0.6, 4, 8), (700, 0.3, 20, 8), (1500, 0.4, 8, 8), (400, 0.2, 12, 8)]
+ONLINE_CASES += [(K, 0.3, 6, D) for D in (4, 8) for K in (257, 512, 513, 1024, 1025, 2048, 2049, 4096)]
+
+
+@pytest.mark.parametrize("K,seconds,passes,D", ONLINE_CASES)
+def test_online_kmeans_bit_exact(ctx, oracle, K, seconds, passes, D):
+    """k_online (and k_online_warp for K <= 256) with its filter and scoring every centroid exactly
+    (GSC_DBG_ONLINE_EXACT): the oracle bit for bit."""
+    pcm, raw, attr, feat = _features(oracle, seconds, ch=2 if K >= 2048 else 1, cs=D // 2)
+    assert len(feat) > K
     c0, _, _ = oracle.yakmo(feat, K)
     c_ref, l_ref, it_ref, err_ref = oracle.knn_scan_reduce(feat, c0, 3, passes)
-    c_gpu, l_gpu, it_gpu, err_gpu = ctx.knn_scan_reduce(feat, c0, 3, passes)
-    assert it_gpu == it_ref
-    assert np.array_equal(l_gpu, l_ref)
-    assert np.array_equal(c_gpu.view(np.uint32), c_ref.view(np.uint32))
-    assert err_gpu == err_ref
+    for flag in (0, ctx.DBG_ONLINE_EXACT):
+        ctx.set_debug(flag)
+        try:
+            c_gpu, l_gpu, it_gpu, err_gpu = ctx.knn_scan_reduce(feat, c0, 3, passes)
+        finally:
+            ctx.set_debug(0)
+        assert it_gpu == it_ref, flag
+        assert np.array_equal(l_gpu, l_ref), flag
+        assert np.array_equal(c_gpu.view(np.uint32), c_ref.view(np.uint32)), flag
+        assert err_gpu == err_ref, flag
 
 
 @pytest.mark.parametrize("K,seconds,passes,D", [(256, 0.25, 100, 8), (100, 0.1, 9, 8), (33, 0.1, 30, 8), (200, 0.15, 12, 4)])
