@@ -310,7 +310,8 @@ int gsc_ctx_set_debug(gsc_ctx *ctx, unsigned flags);
 int gsc_selftest_divider_division(gsc_ctx *ctx, int bits, uint64_t *mismatches);
 /* Debug: counters of the last online k-means launch, 16 x uint64 per frame:
  * batches, points, re-filtered points, resolver rounds, full candidate lists,
- * candidates (lane 0); rest reserved (zero).  After a kmeans_mode 3 k-means (all passes):
+ * candidates (lane 0), commits of a centroid already moved in the same batch; slots 8..15
+ * are zero except in debug builds (GSC_ONLINE_CHECKS, GSC_ONLINE_TIMING).  After a kmeans_mode 3 k-means (all passes):
  * speculation rounds, points committed, lane searches, visit lists that overflowed. */
 int gsc_debug_online_counters(gsc_ctx *ctx, unsigned long long *out, int n_frames);
 /* Debug: counters of the last seeding launch, 8 x uint64 per frame: cycles of seed pick, distance pass,

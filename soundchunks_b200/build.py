@@ -27,14 +27,16 @@ def stale() -> bool:
     return any(os.path.getmtime(os.path.join(CSRC, d)) > t for d in DEPS)
 
 
-def build_variant(out: str, maxrreg: int, checks: bool = False) -> list:
+def build_variant(out: str, maxrreg: int, checks: bool = False, timing: bool = False) -> list:
     """Debug build with a register cap (tools/spill_probe.py): the online k-means shapes then spill on purpose, to
-    show that the results do not depend on the register allocation.  Returns the spilling k_online shapes."""
+    show that the results do not depend on the register allocation.  `checks`: GSC_ONLINE_CHECKS; `timing`:
+    GSC_ONLINE_TIMING (tools/online_serial.py).  Returns the spilling k_online shapes."""
     cmd = [nvcc_path(), "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
            "-fmad=false", "-Xcompiler", "-fPIC,-O2,-fvisibility=default", "-shared", "-o", out,
            "-Xptxas", "-v"]
     cmd += [f"-DGSC_ONLINE_MAXNREG={maxrreg}"] if maxrreg else []
     cmd += ["-DGSC_ONLINE_CHECKS"] if checks else []
+    cmd += ["-DGSC_ONLINE_TIMING"] if timing else []
     cmd += [os.path.join(CSRC, s) for s in SOURCES] + ["-lcudart"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:

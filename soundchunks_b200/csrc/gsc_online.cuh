@@ -98,6 +98,7 @@ __device__ __forceinline__ void gsc_sts_f4(unsigned a, float4 v) {
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
 __device__ __forceinline__ void gsc_atoms_or(unsigned a, unsigned v) { asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ void gsc_atoms_min_u64(unsigned a, unsigned long long v) { asm volatile("red.shared.min.u64 [%0], %1;" ::"r"(a), "l"(v) : "memory"); }
 __device__ __forceinline__ int gsc_atoms_add(unsigned a, int v) { int o; asm volatile("atom.shared.add.s32 %0, [%1], %2;" : "=r"(o) : "r"(a), "r"(v) : "memory"); return o; }
 
 __device__ __forceinline__ int gsc_lds_u8(unsigned a) { unsigned v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return (int)v; }
@@ -208,11 +209,14 @@ struct GscOnLayout {
     static constexpr unsigned MOVED = XHI + (T / 32) * GSC_ON_B * 4;  // int   [B] distinct centroids moved in this batch
     static constexpr unsigned ROWS = MOVED + GSC_ON_B * 4;            // float [B][D]
     static constexpr unsigned WS = ROWS + GSC_ON_B * D * 4;           // int   [B]
-    static constexpr unsigned ETB = WS + GSC_ON_B * 4;                // float [2][B]
+    static constexpr unsigned ETB = WS + GSC_ON_B * 4;                // float [2][B] distances of the committed points
     static constexpr unsigned WKEY = ETB + 2 * GSC_ON_B * 4;          // u64   [B][W] re-filter minima per (request, warp)
-    static constexpr unsigned FK = WKEY + GSC_ON_B * (T / 32) * 8;    // u64   [B(u)][B(lane)] fresh keys of a round
+    // u64 [W][UW][B(lane)] fresh keys of a round as running minima: warp w scores rows u = t0+w+i*W (i < UW = B/W
+    // rounded up), entry [w][i][lane] is the minimum over the first i+1 of them (W * UW * B * 8 = 8 KB for W = 2, 4, 8)
+    static constexpr unsigned FK = WKEY + GSC_ON_B * (T / 32) * 8;
     static constexpr unsigned KEYS = FK + GSC_ON_B * GSC_ON_B * 8;    // u64   [B] proposals of a round
-    static constexpr unsigned CB = KEYS + GSC_ON_B * 8;               // u32   [B] conflict ballots per row u
+    static constexpr unsigned ABEST = KEYS + GSC_ON_B * 8;            // u64   [B] best key of each point's stored list entries
+    static constexpr unsigned CB = ABEST + GSC_ON_B * 8;              // u32   [B] conflict ballots per row u
     static constexpr unsigned DIRTY = CB + GSC_ON_B * 4;              // u32   [T] moved centroids per owner thread
     static constexpr unsigned EPTS = DIRTY + T * 4;                   // int   [B] points to re-filter
     static constexpr unsigned ETHRS = EPTS + GSC_ON_B * 4;            // float [B] ... and their thresholds
@@ -241,6 +245,17 @@ struct GscOnLayout {
 #else
 #define GSC_CHK(cond) ((void)0)
 #endif
+// GSC_ONLINE_TIMING (timing builds of tools/online_serial.py only): warp 0 takes clock() at the borders of its
+// sections and thread 0 adds the cycles of each, per pass, to the launch's debug buffer (slots 10..15):
+//   10 (a) bar 1 -> first bar 2: batch open + the first round's proposals      11 (b) R3 commit
+//   12 (c) R3 take-over of fresh keys, moved checks, list re-scans               13 (d) R3' + R1 of the later rounds
+//   14 (e) bar 2 -> bar 3: R2 (all warps) and both barriers                       15 (f) the whole batch
+// (a)..(d) are the sections in which warp 0 alone issues while the other warps wait at bar 2.
+#ifdef GSC_ONLINE_TIMING
+#define GSC_TM(i) do { const unsigned tm_n = (unsigned)clock(); tm_acc[i] += tm_n - tm_t; tm_t = tm_n; } while (0)
+#else
+#define GSC_TM(i) ((void)0)
+#endif
 // GSC_ONLINE_MAXNREG (debug builds of tools/spill_probe.py only): cap the registers below what the kernel needs, so
 // that ptxas spills -- the results must not change.
 #ifdef GSC_ONLINE_MAXNREG
@@ -267,6 +282,8 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
     constexpr int W = T / 32;
     constexpr int KP = T * CPT;
     constexpr int B = GSC_ON_B, L = GSC_ON_L;
+    constexpr int UW = (B + W - 1) / W;        // rows a warp scores in a round of R2
+    static_assert(W * UW * B <= B * B, "running minima of the fresh keys fit the FK region");
     constexpr unsigned FULL = 0xffffffffu;
     extern __shared__ __align__(16) unsigned char smraw[];
     const unsigned sb = gsc_opaque(gsc_smem_u32(smraw));
@@ -321,14 +338,17 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
     float c0lo = INFINITY, c0hi = -INFINITY;             // exact range of this thread's c0 values (NaN ignored)
     for (int j = tid; j < KP / 4; j += T) gsc_sts_i(sb + Ly::MFLAG + 4u * j, 0);
     gsc_sts_i(sb + Ly::DIRTY + 4u * tid, 0);
-    if (tid < B) gsc_sts_i(sb + Ly::LISTN + 4u * tid, 0);
+    if (tid < B) { gsc_sts_i(sb + Ly::LISTN + 4u * tid, 0); gsc_sts_u64(sb + Ly::ABEST + 8u * tid, GSC_KNONE); }
     if (tid == 0) {
         gsc_sts_d(sb + Ly::ERR, iter0 > 0 ? err_out[f.slot] : 3.40282346638528860e+38);
         gsc_sts_i(sb + Ly::STOP, 0); gsc_sts_i(sb + Ly::MODE, GSC_MODE_DONE);
     }
     __syncthreads();
 
-    unsigned long long c_batches = 0, c_exh = 0, c_rounds = 0, c_over = 0, c_points = 0, c_cands = 0;
+    unsigned long long c_batches = 0, c_exh = 0, c_rounds = 0, c_over = 0, c_points = 0, c_cands = 0, c_again = 0;
+#ifdef GSC_ONLINE_TIMING
+    unsigned tm_acc[6] = {0, 0, 0, 0, 0, 0}, tm_t = 0, tm_f = 0;
+#endif
     int iter = iter0;
     for (;;) {
         // The reference keeps cnts[2][K]: a pass reads cnts[not Odd(iter)] (the previous pass's hits + 1) for the
@@ -342,7 +362,7 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
             gsc_sts_i(cnt_cur + 4u * j, 1);
         }
         __syncthreads();
-        double e_run = 0.0;   // thread 32: enc:743 Double sum in point order, one batch behind the resolver
+        double e_run = 0.0;   // warp 1 (thread 32's copy is used): enc:743 Double sum in point order, one batch behind the resolver
         int nbatch = 0, prev_nb = 0;
 
         for (int base = 0; base < N; base += GSC_ON_TP) {
@@ -449,6 +469,9 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
 
             for (int pos = 0; pos < tn; pos += B) {
                 const int nb = min(B, tn - pos);
+#ifdef GSC_ONLINE_TIMING
+                tm_f = (unsigned)clock();
+#endif
                 // ============ phase 0: refresh the filter copy of this thread's moved centroids ============
                 {
                     const unsigned dirty = (unsigned)gsc_lds_i(sb + Ly::DIRTY + 4u * cell);
@@ -537,7 +560,10 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                     if (d == d) {
                         const unsigned long long kk = gsc_pack(__float_as_uint(d), idword(slot));
                         const int sl = gsc_atoms_add(sb + Ly::LISTN + 4u * b, 1);   // ~3 candidates per point: no contention
-                        if (sl < L) gsc_sts_u64(sb + Ly::LIST + (unsigned)(sl * B + b) * 8u, kk);   // [slot][point]: the resolver's lanes read without bank conflicts
+                        if (sl < L) {   // [slot][point]: the resolver's lanes read without bank conflicts
+                            gsc_sts_u64(sb + Ly::LIST + (unsigned)(sl * B + b) * 8u, kk);
+                            gsc_atoms_min_u64(sb + Ly::ABEST + 8u * (unsigned)b, kk);   // the resolver opens the batch with one load
+                        }
                     }
                 };
                 int qn = 0;   // entries in the warp's queue (warp-uniform)
@@ -640,10 +666,18 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                     }
                 }
                 __syncthreads();   // ---- bar 1: candidate lists complete ----
-                // thread 32 adds the error terms of the previous batch while warp 0 opens this one
-                if (tid == 32 && prev_nb) {
+#ifdef GSC_ONLINE_TIMING
+                tm_t = (unsigned)clock();
+#endif
+                // warp 1 adds the error terms of the previous batch while warp 0 opens this one: lane p takes point p's
+                // sqrt(d / D) (the resolver only stores the distances, so the division and square root stay off its
+                // path), then the terms are added in point order from registers.  Warp 1 has to be back at bar 2 before
+                // warp 0 gets there; 32 dependent shared-memory loads, or 32 square roots on one thread, are not.
+                if (warp == 1 && prev_nb) {
                     const unsigned eb = sb + Ly::ETB + (unsigned)(((nbatch - 1) & 1) * B) * 4u;
-                    for (int p = 0; p < prev_nb; ++p) e_run += (double)gsc_lds_f(eb + 4u * p);
+                    const double t = (lane < prev_nb) ? (double)sqrtf(gsc_lds_f(eb + 4u * lane) / (float)D) : 0.0;   // enc:743
+#pragma unroll
+                    for (int p = 0; p < B; ++p) e_run += __shfl_sync(FULL, t, p);   // (+ 0.0 past the batch's end is exact)
                 }
                 // ============ phase 2: the batch is resolved in rounds ============
                 // warp 0 lane state: abest = best key among the list entries whose centroid has not moved
@@ -673,24 +707,47 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                 };
                 if (warp == 0 && lane < nb) {
                     nl = gsc_lds_i(sb + Ly::LISTN + 4u * lane);
+                    abest = gsc_lds_u64(sb + Ly::ABEST + 8u * lane);   // no centroid has moved yet: the list's minimum
                     over = (nl > L) | force_exact;
                     if (tid == 0) { c_cands += nl; c_over += nl > L; }
                     nl = min(nl, L);
-                    abest = scan_list(false);
+                    GSC_CHK(abest == scan_list(false));
                 }
                 const unsigned etb = sb + Ly::ETB + (unsigned)((nbatch & 1) * B) * 4u;
                 for (;;) {
                     if (warp == 0) {
+#ifdef GSC_ONLINE_TIMING
+                        const int tm_sec = (pending == GSC_MODE_DONE) ? 0 : 3;   // first round of the batch: (a)
+#endif
                         if (pending == GSC_MODE_SCAN) {
                             // ---- R3: first conflicting lane, commit the lanes before it ----
-                            unsigned firstc = 32u;
-                            if (lane >= t0 && lane < nb) {
-                                const unsigned cb = (unsigned)gsc_lds_i(sb + Ly::CB + 4u * lane);
-                                if (cb) firstc = (unsigned)(__ffs(cb) - 1);
+                            // Warp 0 alone issues here while the other warps wait at bar 2, and the shared-memory accessors
+                            // keep source order: every load the section can issue early goes out in one trip before the
+                            // commit's stores.  The committing lanes' winners are distinct (a repeated winner is a conflict),
+                            // so their hit counts and moved flags are read before any of them is written.
+                            const bool act = lane >= t0 && lane < nb;
+                            unsigned cb = 0;
+                            int cntw = 0, already = 0;
+                            if (act) {
+                                cb = (unsigned)gsc_lds_i(sb + Ly::CB + 4u * lane);
+                                cntw = gsc_lds_i(cnt_cur + 4u * w);
+                                already = gsc_lds_u8(sb + Ly::MFLAG + (unsigned)w);
                             }
-                            const int tstar = min(nb, (int)__reduce_min_sync(FULL, firstc));
+                            const int tstar = min(nb, (int)__reduce_min_sync(FULL, cb ? (unsigned)(__ffs(cb) - 1) : 32u));
                             const bool commit = lane >= t0 && lane < tstar;
-                            int already = 0;
+                            const bool takes = lane >= tstar && lane < nb;
+                            if (takes) {
+                                // unresolved lanes take over the fresh keys of the committed rows t0 .. tstar-1: warp ww of R2
+                                // scored rows t0+ww, t0+ww+W, ... and stored running minima, so one entry per warp covers them
+                                unsigned long long kq[W];
+#pragma unroll
+                                for (int ww = 0; ww < W; ++ww) {
+                                    const int n = (tstar - t0 - ww + W - 1) / W;   // rows of warp ww below tstar (tstar > t0)
+                                    kq[ww] = (n > 0) ? gsc_lds_u64(sb + Ly::FK + (unsigned)((ww * UW + n - 1) * B + lane) * 8u) : GSC_KNONE;
+                                }
+#pragma unroll
+                                for (int ww = 0; ww < W; ++ww) if (kq[ww] < fresh) fresh = kq[ww];
+                            }
                             if (commit) {
                                 GSC_CHK(w >= 0 && w < KP && gsc_lds_u16(sb + Ly::S2O + 2u * (unsigned)w) < K && base + pos + lane < N);
                                 gsc_sts_row<D>(sb + Ly::C + (unsigned)w * D * 4, rn);
@@ -700,14 +757,14 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                                     for (int k = 0; k < DF; ++k) nc = fmaf(rn[k], rn[k], nc);
                                     gsc_sts_f(sb + Ly::H + 4u * (unsigned)w, -0.5f * nc * (1.0f - GSC_ON_G));
                                 }
-                                gsc_sts_i(cnt_cur + 4u * w, gsc_lds_i(cnt_cur + 4u * w) + 1);            // enc:744
-                                lab[base + pos + lane] = w;                                               // enc:742
-                                gsc_sts_f(etb + 4u * lane, sqrtf(__uint_as_float(gsc_kd(key)) / (float)D));  // enc:743 (term)
-                                already = gsc_lds_u8(sb + Ly::MFLAG + (unsigned)w);
+                                gsc_sts_i(cnt_cur + 4u * w, cntw + 1);                // enc:744
+                                lab[base + pos + lane] = w;                           // enc:742
+                                gsc_sts_i(etb + 4u * lane, (int)gsc_kd(key));         // enc:743: the distance (thread 32 takes the term)
                                 gsc_sts_u8(sb + Ly::MFLAG + (unsigned)w, already ? 2 : 1);   // 2: moved again in this round
                                 gsc_atoms_or(sb + Ly::DIRTY + 4u * (unsigned)(w / CPT), 1u << (w % CPT));
                             }
                             const unsigned anyal = __ballot_sync(FULL, commit && already);
+                            if (tid == 0) c_again += __popc(anyal);
                             {   // the moved list holds every centroid once
                                 const unsigned newm = __ballot_sync(FULL, commit && !already);
                                 if (commit && !already) gsc_sts_i(sb + Ly::MOVED + 4u * (unsigned)(nm + __popc(newm & ((1u << lane) - 1u))), w);
@@ -715,17 +772,12 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                                 GSC_CHK(nm <= B);
                             }
                             __syncwarp();
-                            // unresolved lanes take over the fresh keys of the committed rows
-                            if (lane >= tstar && lane < nb) {
-                                for (int u = t0; u < tstar; u += 4) {   // 4 independent loads per step
-                                    unsigned long long kq[4];
-#pragma unroll
-                                    for (int q = 0; q < 4; ++q)
-                                        kq[q] = (u + q < tstar) ? gsc_lds_u64(sb + Ly::FK + (unsigned)((u + q) * B + lane) * 8u) : GSC_KNONE;
-#pragma unroll
-                                    for (int q = 0; q < 4; ++q) if (kq[q] < fresh) fresh = kq[q];
-                                }
-                                if (anyal && fresh != GSC_KNONE && gsc_lds_u8(sb + Ly::MFLAG + gsc_ks(fresh)) == 2) {
+                            GSC_TM(1);
+                            if (takes) {
+                                // both moved flags in one trip (after the commit's stores)
+                                const int mvf = (anyal && fresh != GSC_KNONE) ? gsc_lds_u8(sb + Ly::MFLAG + gsc_ks(fresh)) : 0;
+                                const int mva = (abest != GSC_KNONE) ? gsc_lds_u8(sb + Ly::MFLAG + gsc_ks(abest)) : 0;
+                                if (mvf == 2) {
                                     // this lane's best moved centroid moved again: its key is stale, rebuild from the moved list
                                     // (the other lanes' minima are over centroids that did not move again and stay valid)
                                     fresh = GSC_KNONE;
@@ -737,7 +789,7 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                                         if (d == d) { const unsigned long long kk = gsc_pack(__float_as_uint(d), idword(id)); if (kk < fresh) fresh = kk; }
                                     }
                                 }
-                                if (abest != GSC_KNONE && gsc_lds_u8(sb + Ly::MFLAG + gsc_ks(abest))) {
+                                if (mva) {
                                     // the leader among the unmoved centroids moved
                                     if (exact) { exact = 0; over = 1; abest = GSC_KNONE; }   // no list behind it: re-filter again
                                     else abest = scan_list(true);
@@ -748,6 +800,7 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                                 if (commit && already) gsc_sts_u8(sb + Ly::MFLAG + (unsigned)w, 1);
                             }
                             t0 = tstar;
+                            GSC_TM(2);
                         } else if (pending == GSC_MODE_REFILTER) {
                             // ---- R3': every re-filtered lane now knows its exact best unmoved centroid ----
                             if ((badmask >> lane) & 1u) {
@@ -777,6 +830,7 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                             GSC_CHK(gsc_lds_i(sb + Ly::LISTN + 4u * lane) >= 0);
                             if (lane < nm) gsc_sts_u8(sb + Ly::MFLAG + (unsigned)gsc_lds_i(sb + Ly::MOVED + 4u * lane), 0);
                             gsc_sts_i(sb + Ly::LISTN + 4u * lane, 0);
+                            gsc_sts_u64(sb + Ly::ABEST + 8u * lane, GSC_KNONE);
                             if (lane == 0) gsc_sts_i(sb + Ly::MODE, GSC_MODE_DONE);
                             pending = GSC_MODE_DONE;
                             ++c_batches; c_points += nb;
@@ -812,13 +866,13 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                                 pending = GSC_MODE_SCAN;
                             }
                         }
+                        GSC_TM(tm_sec);
                     }
                     __syncthreads();   // ---- bar 2: proposals / request visible ----
                     const int mode = gsc_lds_i(sb + Ly::MODE);
                     if (mode == GSC_MODE_DONE) break;
                     if (mode == GSC_MODE_SCAN) {
                         // ---- R2: lane t scores the proposed rows u (warp w takes u = t0+w, t0+w+W, ...) ----
-                        constexpr int UW = (B + W - 1) / W;
                         const int s0 = gsc_lds_i(sb + Ly::T0);
                         const unsigned long long mykey = gsc_lds_u64(sb + Ly::KEYS + 8u * lane);
                         const int myw = gsc_lds_i(sb + Ly::WS + 4u * lane);
@@ -830,13 +884,15 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                             wu[i] = -2;
                             if (u < nb) { wu[i] = gsc_lds_i(sb + Ly::WS + 4u * u); gsc_lds_row<D>(sb + Ly::ROWS + (unsigned)u * D * 4, ru[i]); }
                         }
+                        unsigned long long run = GSC_KNONE;
 #pragma unroll
                         for (int i = 0; i < UW; ++i) {
                             const int u = s0 + warp + i * W;
                             if (u < nb) {   // uniform per warp
                                 const float d = gsc_ann_dist<D>(xb, ru[i]);
                                 const unsigned long long kk = (d == d) ? gsc_pack(__float_as_uint(d), (unsigned)wu[i]) : GSC_KNONE;
-                                gsc_sts_u64(sb + Ly::FK + (unsigned)(u * B + lane) * 8u, kk);
+                                if (kk < run) run = kk;
+                                gsc_sts_u64(sb + Ly::FK + (unsigned)((warp * UW + i) * B + lane) * 8u, run);
                                 const bool conf = (lane > u) && (lane < nb) && ((wu[i] == myw) || (kk < mykey));
                                 const unsigned cb = __ballot_sync(FULL, conf);
                                 if (lane == 0) gsc_sts_i(sb + Ly::CB + 4u * u, (int)cb);
@@ -874,7 +930,11 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
                         }
                     }
                     __syncthreads();   // ---- bar 3: round results complete ----
+                    GSC_TM(4);
                 }
+#ifdef GSC_ONLINE_TIMING
+                tm_acc[5] += (unsigned)clock() - tm_f;
+#endif
                 prev_nb = nb;
                 ++nbatch;
             }
@@ -882,10 +942,17 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
         // ---- end of pass: enc:754-761 ----
         __syncthreads();
         ++iter;
+#ifdef GSC_ONLINE_TIMING
+        if (tid == 0 && dbg) {   // per pass: 32-bit sums do not wrap
+            unsigned long long *o = dbg + (long long)f.slot * 16 + 10;
+#pragma unroll
+            for (int i = 0; i < 6; ++i) { o[i] += tm_acc[i]; tm_acc[i] = 0; }
+        }
+#endif
         if (tid == 32) {
             if (prev_nb) {
                 const unsigned eb = sb + Ly::ETB + (unsigned)(((nbatch - 1) & 1) * B) * 4u;
-                for (int p = 0; p < prev_nb; ++p) e_run += (double)gsc_lds_f(eb + 4u * p);
+                for (int p = 0; p < prev_nb; ++p) e_run += (double)sqrtf(gsc_lds_f(eb + 4u * p) / (float)D);   // enc:743
             }
             gsc_sts_d(sb + Ly::ERR, e_run);
             const bool same = (e_run > prevErr) ? ((e_run - prevErr) <= tol) : ((prevErr - e_run) <= tol);
@@ -916,7 +983,7 @@ __global__ void GSC_ONLINE_BOUNDS(T) k_online(const GscFrame *__restrict__ frame
         done[f.slot] = gsc_lds_i(sb + Ly::STOP);
         if (dbg) {
             unsigned long long *o = dbg + (long long)f.slot * 16;
-            o[0] += c_batches; o[1] += c_points; o[2] += c_exh; o[3] += c_rounds; o[4] += c_over; o[5] += c_cands;
+            o[0] += c_batches; o[1] += c_points; o[2] += c_exh; o[3] += c_rounds; o[4] += c_over; o[5] += c_cands; o[6] += c_again;
         }
     }
 }
